@@ -2,9 +2,11 @@
 """bench.py -- env-steps/s of the batched Dojo step on B200 (BASELINE.json metric: forward and forward+gradient).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--mech ant|quadruped|atlas|pendulum] [--batch B] [--mode fwd|grad] [--no-sub]
+                    [--mech ant|quadruped|atlas|pendulum] [--batch B] [--mode fwd|grad] [--no-sub] [--dump-outputs DIR]
 
-One JSON line is printed by rank 0.
+One JSON line is printed by rank 0.  With --dump-outputs, rank 0 also writes what the last timed step of each record returned
+(next states, status, Newton iterations and, in grad mode, the gradients; see last_step_outputs) as .npy files, so that two builds
+can be compared output for output: the states and inputs are seeded, identical from run to run.
 
 Headline (`value`, `e2e`, `roofline`, `cpu_baseline`, `parity`) = BASELINE.json configs[1]: Ant (DojoEnvironments defaults),
 batch 4096 per GPU, forward-only step!.  With no --mech / --batch / --mode flags the same line also carries `sub_records`, so that one
@@ -95,6 +97,29 @@ def synthetic_batch(mech, B, seed, name=None):
             protos[e].reshape(mech.Nb, 13)[:, 2] += rng.uniform(*w["ground"]) - min_clearance(mech, protos[e])
     Z = protos[rng.integers(0, n_proto, B)].copy()
     return Z, rng
+
+
+DUMP_BYTES_PER_RECORD = 15_000_000  # --dump-outputs: the headline and at most three sub-records stay under 64 MB in all
+
+
+def last_step_outputs(z_next, status, iters, Fz=None, Fu=None, budget=DUMP_BYTES_PER_RECORD):
+    """What a caller of the timed step received from the last timed step, as float64 host arrays: next states, status and Newton
+    iterations of every environment, or of a fixed seeded sample of them where that would exceed half of `budget`; the gradients
+    (grad mode) of a fixed seeded sample of environments that fits in the other half."""
+    import torch
+    B = z_next.shape[0]
+
+    def rows(per_env, seed):
+        n = min(B, max(1, budget // 2 // per_env))
+        sel = np.arange(B) if n == B else np.sort(np.random.default_rng(seed).choice(B, size=n, replace=False))
+        return torch.from_numpy(sel).to(z_next.device)
+
+    sel = rows(8 * (z_next.shape[1] + 2), 11)
+    out = {"z_next": z_next[sel], "status": status[sel], "iters": iters[sel]}
+    if Fz is not None:
+        gsel = rows(8 * (Fz[0].numel() + Fu[0].numel()), 12)
+        out.update(Fz=Fz[gsel], Fu=Fu[gsel])
+    return {k: v.double().cpu().numpy() for k, v in out.items()}
 
 
 def random_inputs(mech, rng, T, B, scale):
@@ -228,7 +253,8 @@ def ncu_summary(mech_name, mode):
 
 
 # ---------------------------------------------------------------------------------------------------- one configuration on the GPU(s)
-def run_config(name, B, mode, steps, warmup, rank, local_rank, world, dist, threads, quota, headline, e2e_steps=10, cpu_sample=2048, sample_clocks=True):
+def run_config(name, B, mode, steps, warmup, rank, local_rank, world, dist, threads, quota, headline, e2e_steps=10, cpu_sample=2048, sample_clocks=True,
+               outputs=None):
     import torch
     from dojo_jl_b200.solver import BatchedStepper
     mech = dj.get_mechanism(name)
@@ -326,6 +352,8 @@ def run_config(name, B, mode, steps, warmup, rank, local_rank, world, dist, thre
     ms_per_step = total_ms / steps
     value = world * B / (ms_per_step * 1e-3)
     Z_final_stepwise = Za.clone()
+    if outputs is not None:  # --dump-outputs
+        outputs.update(last_step_outputs(Za, status, iters, *((Fz, Fu) if mode == "grad" else ())))
 
     what = "forward-only step!" if mode == "fwd" else "step! + get_maximal_gradients"
     rec = {"workload": f"{name} (DojoEnvironments defaults, h={mech.timestep}) batch={B}/GPU {what}", "mechanism": name, "batch_per_gpu": B, "global_batch": B * world,
@@ -475,7 +503,11 @@ def main():
     ap.add_argument("--mode", default=None, choices=["fwd", "grad"])
     ap.add_argument("--no-sub", action="store_true", help="headline record only")
     ap.add_argument("--cpu-threads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of every record returned to DIR/<record>.<array>.npy (float64, < 64 MB in all)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3)
     custom = args.mech is not None or args.batch is not None or args.mode is not None
     name, B, mode = args.mech or "ant", args.batch or 4096, args.mode or "fwd"
@@ -545,7 +577,9 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
 
-    head = run_config(name, B, mode, args.steps, args.warmup, rank, local_rank, world, dist, threads, quota, headline=True)
+    dumps = {} if args.dump_outputs else None
+    head = run_config(name, B, mode, args.steps, args.warmup, rank, local_rank, world, dist, threads, quota, headline=True,
+                      outputs=None if dumps is None else dumps.setdefault("headline", {}))
     subs = {}
     if not custom and not args.no_sub:
         ksub, wsub = min(args.steps, 10), 3
@@ -556,7 +590,8 @@ def main():
         for key, n2, b2, m2 in plan:
             try:
                 r = run_config(n2, b2, m2, ksub, wsub, rank, local_rank, world, dist, threads, quota, headline=False, e2e_steps=2,
-                               cpu_sample=512 if n2 != "atlas" else 128, sample_clocks=False)
+                               cpu_sample=512 if n2 != "atlas" else 128, sample_clocks=False,
+                               outputs=None if dumps is None else dumps.setdefault(key, {}))
                 subs[key] = r
             except Exception as ex:  # a sub-record must never take the headline down
                 subs[key] = {"error": f"{type(ex).__name__}: {ex}"}
@@ -571,6 +606,11 @@ def main():
             "mean_newton_iters": head["mean_newton_iters"], "failed_env_steps": head["failed_env_steps"], "failed_rate": head["failed_rate"],
             "shared_bytes_per_env": head.get("shared_bytes_per_env"), "gather": head.get("gather"), "step_ms_min_max": head["step_ms_min_max"],
             "sub_records": subs}
+    if dumps is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for rec_name, arrays in dumps.items():
+            for arr_name, a in arrays.items():
+                np.save(os.path.join(args.dump_outputs, f"{rec_name}.{arr_name}.npy"), a)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
